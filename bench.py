@@ -42,6 +42,27 @@ ALG_BYTES_PER_POINT = 36  # src xyz 12 + matched target xyz 12 + matched normal 
 MAX_DIST = 0.02
 ITERS = 30
 WORKLOAD = "config2: point-to-plane ICP 1M->1M + normals, 30 iters, r=0.02 (SURVEY.md 8d)"
+DUMP_BYTES = 64 << 20  # --dump-outputs: at most this much in all
+
+
+def result_arrays(T, fitness, inlier_rmse, correspondence_set):
+    """what a caller of registration_icp receives (RegistrationResult), as float64 arrays for --dump-outputs"""
+    return {"transformation": np.asarray(T, np.float64).reshape(4, 4), "fitness": np.float64(fitness),
+            "inlier_rmse": np.float64(inlier_rmse), "correspondence_set": np.asarray(correspondence_set, np.float64)}
+
+
+def dump_outputs(path, arrays):
+    """Writes each array as path/<name>.npy.  Should the arrays exceed DUMP_BYTES, every array with more rows than
+    its share keeps a fixed, seeded sample of its rows (ascending), and <name>_rows.npy holds their indices."""
+    os.makedirs(path, exist_ok=True)
+    total = sum(a.nbytes for a in arrays.values())
+    for name, a in list(arrays.items()):
+        if total > DUMP_BYTES and a.ndim > 0 and a.nbytes > DUMP_BYTES // (2 * len(arrays)):
+            keep = max(1, DUMP_BYTES // (2 * len(arrays)) // (a.nbytes // len(a)))
+            rows = np.sort(np.random.default_rng(0).choice(len(a), keep, replace=False))
+            arrays[name], arrays[name + "_rows"] = a[rows], rows.astype(np.float64)
+    for name, a in arrays.items():
+        np.save(os.path.join(path, name + ".npy"), a)
 
 
 def peaks():
@@ -189,7 +210,9 @@ def run_reference(args, rank):
     if rank != 0:
         return
     src, tgt, tn = make_workload(args.points)
-    med, times, r, info = cpu_arm(src, tgt, tn, runs=max(args.steps, 3), budget_s=120.0, warm=min(args.warmup, 1))
+    med, times, r, info = cpu_arm(src, tgt, tn, runs=args.steps, budget_s=float("inf"), warm=min(args.warmup, 1))
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, result_arrays(r["transformation"], r["fitness"], r["inlier_rmse"], r["correspondence_set"]))
     v = ITERS / med
     print(json.dumps({
         "impl": "reference", "metric": "icp_iterations_per_sec", "value": v, "unit": "iter/s", "n_gpus": args.gpus,
@@ -301,6 +324,12 @@ def run_native(args, rank, world):
     resident_steps_ms = list(step_log)
     launches = L.cphb_launch_count() - launches0
     loop_ms, loop_launches = res.loop_ms, res.loop_launches
+    if args.dump_outputs:
+        corr = res.correspondence_set
+        if dist is not None:    # each rank holds the pairs of its block: the caller of N ranks receives all of them
+            from cupoch_b200.distributed import gather_correspondences
+            corr = gather_correspondences(dist, corr, 0, world)
+        outputs = result_arrays(res.transformation, res.fitness, res.inlier_rmse, corr)
 
     # ---- end-to-end through the public API with host (pinned) buffers ---------------------------
     h_src, p1 = pinned_array(L, src_local.shape)
@@ -350,8 +379,8 @@ def run_native(args, rank, world):
     q_pc = cph.geometry.PointCloud(np.ascontiguousarray(src[lo:hi]))   # queries: no collective, shard by index
     for _ in range(2):
         tree.search_radius(q_pc.points, MAX_DIST, 1)
-    knn_ms, _ = timed(lambda: tree.search_radius(q_pc.points, MAX_DIST, 1), max(args.steps, 3))
-    knn_steps = max(args.steps, 3)
+    knn_ms, _ = timed(lambda: tree.search_radius(q_pc.points, MAX_DIST, 1), args.steps)
+    knn_steps = args.steps
     # ---- sub-records (N = 1 only; each a few device milliseconds) -----------------------------------
     extra = {}
     if world == 1 and not args.no_extras:
@@ -361,10 +390,10 @@ def run_native(args, rank, world):
         os.environ["CPHB_CERT_GAIN"] = "0"
         for _ in range(2):
             step_resident()
-        nocert_ms, res_nc = timed(step_resident, max(args.steps, 3))
+        nocert_ms, res_nc = timed(step_resident, args.steps)
         del os.environ["CPHB_CERT_GAIN"]
         assert np.array_equal(res_nc.transformation, res.transformation), "certificates changed the result"
-        extra["certificates_off"] = {"value": ITERS * 1e3 / (nocert_ms / max(args.steps, 3)), "unit": "iter/s",
+        extra["certificates_off"] = {"value": ITERS * 1e3 / (nocert_ms / args.steps), "unit": "iter/s",
                                      "loop_iters_per_sec": ITERS * 1e3 / res_nc.loop_ms,
                                      "note": "same workload, every launch searches (CPHB_CERT_GAIN=0); identical result"}
         # (b) config 3 of BASELINE.json: VoxelDownSample(0.02) + SearchRadius(k=1, r=0.05) on 10 M points
@@ -449,6 +478,8 @@ def run_native(args, rank, world):
         out.update(extra)
         if world == 1 and not args.no_cpu:
             out["cpu_baseline"], out["parity_vs_cpu_baseline"] = cpu_baseline(src, tgt, tn, res_e)
+        if args.dump_outputs:
+            dump_outputs(args.dump_outputs, outputs)
         print(json.dumps(out))
     for p in (p1, p2, p3):
         L.cphb_free_host(p)
@@ -621,7 +652,7 @@ def config3_records(cph, L, timed, peak, args):
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=5)
+    ap.add_argument("--steps", type=int, default=5, help="timed steps of each config-2 leg (the config 3/4/5 sub-records time fixed counts)")
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", default="native", choices=["native", "reference"])
     ap.add_argument("--points", type=int, default=1_000_000)
@@ -635,7 +666,12 @@ def main():
     ap.add_argument("--config5-multi", action="store_true", help="also run the config-5 sub-record at N > 1")
     ap.add_argument("--comm", default="p2p", choices=["p2p", "nccl"],
                     help="N>1 exchange: p2p = peer-memory stores fused into the reduce kernel, nccl = ncclAllReduce")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the result of the last timed registration (transformation, fitness, inlier_rmse, "
+                         "correspondence_set) as DIR/<name>.npy in float64")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     args.warmup = max(args.warmup, 3) if args.impl == "native" else args.warmup
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
