@@ -6,7 +6,8 @@
 
 Mirrors `import cupoch as cph` for: cph.geometry.{PointCloud, KDTreeFlann, KDTreeSearchParamKNN,
 KDTreeSearchParamRadius, VoxelGrid, OccupancyGrid, OccupancyVoxel}, cph.registration.{registration_icp,
-registration_generalized_icp, registration_colored_icp, ICPConvergenceCriteria, TransformationEstimation*
+registration_generalized_icp, registration_colored_icp, registration_fast_based_on_feature_matching,
+FastGlobalRegistrationOption, ICPConvergenceCriteria, TransformationEstimation*
 (user subclasses run the generic loop), RegistrationResult, compute_fpfh_feature, kabsch, kabsch_weighted},
 cph.utility.{Vector3fVector, compute_jtj_jtr, compute_weighted_jtj_jtr}; cupoch_b200.distributed holds the
 multi-GPU orchestration (torch.distributed).  All computation runs in libcupoch_b200.so (hand-written sm_100a CUDA);

@@ -43,6 +43,12 @@ class OccGridParams(C.Structure):
                 ("prob_miss_log", C.c_float), ("occ_prob_thres_log", C.c_float)]
 
 
+class FgrOption(C.Structure):
+    _fields_ = [("division_factor", C.c_float), ("use_absolute_scale", C.c_int), ("decrease_mu", C.c_int),
+                ("maximum_correspondence_distance", C.c_float), ("iteration_number", C.c_int),
+                ("tuple_scale", C.c_float), ("maximum_tuple_count", C.c_int)]
+
+
 _P = C.c_void_p
 _F3 = C.POINTER(C.c_float)
 _I3 = C.POINTER(C.c_int32)
@@ -112,6 +118,12 @@ _SIGNATURES = {
     "cphb_compute_weighted_jtj_jtr": (C.c_int, [_P, _P, C.c_size_t, C.c_int, C.c_float, C.c_float, C.POINTER(C.c_double),
                                                  C.POINTER(C.c_float), _P]),
     "cphb_compute_fpfh_feature": (C.c_int, [_P, _P, C.c_size_t, C.c_int, C.c_float, C.c_int, _P, _P]),
+    "cphb_fgr_default_option": (None, [C.POINTER(FgrOption)]),
+    "cphb_feature_nn": (C.c_int, [_P, C.c_size_t, _P, C.c_size_t, C.c_int, _P, _P, _P, _P, _P]),
+    "cphb_fgr_advanced_matching": (C.c_int, [_P, C.c_size_t, _P, C.c_size_t, _P, C.c_size_t, _P, C.c_size_t, C.c_int,
+                                             C.POINTER(FgrOption), _P, C.POINTER(C.c_int64), _P]),
+    "cphb_fast_global_registration": (C.c_int, [C.POINTER(Cloud), C.POINTER(Cloud), _P, C.c_size_t, _P, C.c_size_t,
+                                                C.c_int, C.POINTER(FgrOption), C.POINTER(IcpResult), _P, _P, _P]),
     "cphb_cluster_dbscan": (C.c_int, [_P, C.c_size_t, C.c_float, C.c_int, C.c_int, _P, C.POINTER(C.c_int), _P]),
     "cphb_reserve_pool": (C.c_int, [C.c_size_t]),
     "cphb_malloc": (_P, [C.c_size_t]),

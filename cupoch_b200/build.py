@@ -20,7 +20,7 @@ SRC = os.path.join(HERE, "csrc")
 OBJ = os.path.join(SRC, "_build")
 LIB = os.path.join(HERE, "lib", "libcupoch_b200.so")
 SOURCES = ["index.cu", "sort.cu", "search.cu", "icp.cu", "voxel.cu", "features.cu", "filters.cu", "voxelgrid.cu", "comm.cu",
-           "reduce.cu", "fpfh.cu", "cluster.cu", "occgrid.cu"]
+           "reduce.cu", "fpfh.cu", "cluster.cu", "occgrid.cu", "fgr.cu"]
 NVCC = os.environ.get("NVCC", "/usr/local/cuda/bin/nvcc")
 FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-O3", "-lineinfo", "-std=c++17", "-fmad=false",
          "-Xcompiler", "-fPIC", "-I" + os.path.join(ROOT, "include"), "-I" + SRC]

@@ -1,5 +1,6 @@
-"""cupoch.registration mirror (ICP subset): registration_icp / registration_generalized_icp /
-registration_colored_icp, ICPConvergenceCriteria, TransformationEstimation*, RegistrationResult.
+"""cupoch.registration mirror: registration_icp / registration_generalized_icp / registration_colored_icp,
+registration_fast_based_on_feature_matching, ICPConvergenceCriteria, TransformationEstimation*,
+FastGlobalRegistrationOption, RegistrationResult.
 Signatures follow src/python/cupoch_pybind/registration/registration.cpp:62-478.
 """
 import ctypes as C
@@ -373,10 +374,16 @@ def kabsch_weighted(model, target, weight):
 
 
 class Feature:
-    """registration::Feature<33> (feature.h): `data` is [n, 33] float32 on the device; .cpu() downloads it.  (The
-    reference stores it dimension-major for Python; here it is one row per point.)"""
+    """registration::Feature<33> / Feature<352> (feature.h): `data` is [n, dim] float32 on the device; .cpu() downloads
+    it.  (The reference stores it dimension-major for Python; here it is one row per point.)  Besides a DeviceArray,
+    `data` may be anything DeviceArray.wrap accepts -- a numpy array, a torch tensor (CPU or CUDA) -- of shape
+    [n, 33] or [n, 352], so that features computed elsewhere can be handed to the global registration."""
 
     def __init__(self, data):
+        if not isinstance(data, DeviceArray):
+            data = DeviceArray.wrap(data, np.float32)
+            if len(data.shape) != 2 or data.shape[1] not in (33, 352):
+                raise ValueError("Feature: expected [n, 33] or [n, 352], got %s" % (data.shape,))
         self.data = data
 
     def dimension(self):
@@ -407,6 +414,96 @@ def compute_fpfh_feature(input, search_param):
         raise RuntimeError("Unsupport search param type.")
     _lib.check(_lib.lib().cphb_compute_fpfh_feature(input._points.ptr, input._normals.ptr, n, knn, radius, max_nn, out.ptr, None))
     return Feature(out)
+
+
+class FastGlobalRegistrationOption:  # fast_global_registration.h:43-104, registration.cpp:217-276
+    """Options of registration_fast_based_on_feature_matching; defaults are the reference's."""
+
+    def __init__(self, division_factor=1.4, use_absolute_scale=False, decrease_mu=True,
+                 maximum_correspondence_distance=0.025, iteration_number=64, tuple_scale=0.95, maximum_tuple_count=1000):
+        self.division_factor = float(division_factor)
+        self.use_absolute_scale = bool(use_absolute_scale)
+        self.decrease_mu = bool(decrease_mu)
+        self.maximum_correspondence_distance = float(maximum_correspondence_distance)
+        self.iteration_number = int(iteration_number)
+        self.tuple_scale = float(tuple_scale)
+        self.maximum_tuple_count = int(maximum_tuple_count)
+
+    def _c(self):
+        o = _lib.FgrOption()
+        o.division_factor, o.use_absolute_scale, o.decrease_mu = self.division_factor, int(self.use_absolute_scale), int(self.decrease_mu)
+        o.maximum_correspondence_distance, o.iteration_number = self.maximum_correspondence_distance, self.iteration_number
+        o.tuple_scale, o.maximum_tuple_count = self.tuple_scale, self.maximum_tuple_count
+        return o
+
+    def __repr__(self):
+        return ("registration::FastGlobalRegistrationOption with division_factor=%f use_absolute_scale=%d decrease_mu=%d "
+                "maximum_correspondence_distance=%f iteration_number=%d tuple_scale=%f maximum_tuple_count=%d"
+                % (self.division_factor, self.use_absolute_scale, self.decrease_mu, self.maximum_correspondence_distance,
+                   self.iteration_number, self.tuple_scale, self.maximum_tuple_count))
+
+
+def _features(f, n, what):
+    if not isinstance(f, Feature):
+        f = Feature(f)
+    if f.num() != n:
+        raise ValueError("%s: %d features for %d points" % (what, f.num(), n))
+    return f
+
+
+def registration_fast_based_on_feature_matching(source, target, source_feature, target_feature, option=None,
+                                                return_trace=False):
+    """registration::FastGlobalRegistration<33 | 352> (fast_global_registration.cu:391-431).  With return_trace the
+    result also carries `trace` [iteration_number, 4, 4]: the pose in normalised coordinates after every iteration."""
+    option = option or FastGlobalRegistrationOption()
+    _lib.require_gpu()
+    fs = _features(source_feature, len(source), "source_feature")
+    ft = _features(target_feature, len(target), "target_feature")
+    if fs.dimension() != ft.dimension():
+        raise ValueError("source and target features differ in dimension")
+    sc, tc = source._cloud(False), target._cloud(False)
+    res = _lib.IcpResult()
+    corr = _DevicePool.take((max(len(source), 1), 2), np.int32)
+    tr = DeviceArray((max(option.iteration_number, 1), 16), np.float32) if return_trace else None
+    _lib.check(_lib.lib().cphb_fast_global_registration(C.byref(sc), C.byref(tc), fs.data.ptr, fs.num(), ft.data.ptr, ft.num(),
+                                                        fs.dimension(), C.byref(option._c()), C.byref(res), corr.ptr,
+                                                        tr.ptr if tr is not None else None, None))
+    out = _result(res, corr, True)
+    if return_trace:
+        out.trace = tr.cpu(max(option.iteration_number, 0)).reshape(-1, 4, 4)
+    return out
+
+
+def fgr_advanced_matching(source_points, target_points, source_feature, target_feature, option=None):
+    """Test hook (cphb_fgr_advanced_matching): NormalizePointCloud + AdvancedMatching of the reference
+    (fast_global_registration.cu:103-265) -> (pairs [m, 2] int32 (source, target), counts dict)."""
+    option = option or FastGlobalRegistrationOption()
+    _lib.require_gpu()
+    sp, tp = DeviceArray.wrap(source_points), DeviceArray.wrap(target_points)
+    fs, ft = _features(source_feature, len(sp), "source_feature"), _features(target_feature, len(tp), "target_feature")
+    out = DeviceArray((max(option.maximum_tuple_count, 1), 2), np.int32)
+    counts = (C.c_int64 * 4)()
+    _lib.check(_lib.lib().cphb_fgr_advanced_matching(sp.ptr, len(sp), tp.ptr, len(tp), fs.data.ptr, fs.num(), ft.data.ptr,
+                                                     ft.num(), fs.dimension(), C.byref(option._c()), out.ptr, counts, None))
+    return out.cpu(counts[0]), {"pairs": counts[0], "mutual": counts[1], "trials": counts[2], "passing_pairs": counts[3]}
+
+
+def bruteforce_nn(ref, query, both_directions=False):
+    """knn::BruteForceNN<33 | 352>(ref, query, indices, distances) (bruteforce_nn.inl:101-135) on [n, dim] features:
+    -> (indices [m] int32, squared distances [m] float32) of the nearest ref row for every query row.  With
+    both_directions also (indices [n], squared distances [n]) of the nearest query row for every ref row, from the
+    same distance evaluations (the two-way matcher of the global registration)."""
+    _lib.require_gpu()
+    r = ref if isinstance(ref, Feature) else Feature(ref)
+    q = query if isinstance(query, Feature) else Feature(query)
+    dim = r.dimension() if r.dimension() == q.dimension() else -1
+    idx, d2 = DeviceArray((max(q.num(), 1),), np.int32), DeviceArray((max(q.num(), 1),), np.float32)
+    ridx = DeviceArray((max(r.num(), 1),), np.int32) if both_directions else None
+    rd2 = DeviceArray((max(r.num(), 1),), np.float32) if both_directions else None
+    _lib.check(_lib.lib().cphb_feature_nn(r.data.ptr, r.num(), q.data.ptr, q.num(), dim, idx.ptr, d2.ptr,
+                                          ridx.ptr if ridx else None, rd2.ptr if rd2 else None, None))
+    out = (idx.cpu(q.num()), d2.cpu(q.num()))
+    return out + (ridx.cpu(r.num()), rd2.cpu(r.num())) if both_directions else out
 
 
 class IcpContext:

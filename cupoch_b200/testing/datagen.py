@@ -70,3 +70,24 @@ def make_source(target, T_gt, perm_seed, noise_seed, sigma, attrs=()):
             b = (b.astype(np.float64) @ Ti[:3, :3].T)
         out.append(np.ascontiguousarray(b, np.float32))
     return out if len(out) > 1 else out[0]
+
+
+def bumps_scene(n, seed, n_bumps=24, extent=1.0):
+    """A non-periodic surface for global registration: a height field of seeded Gaussian bumps of varied width and
+    height over [0, extent]^2, plus two tilted planes standing on it (float32, [n, 3]).  Unlike surface(), no two
+    neighbourhoods repeat, so local descriptors such as FPFH have unambiguous matches."""
+    rng = np.random.default_rng(seed)
+    c = rng.uniform(0, extent, (n_bumps, 2))
+    h = rng.uniform(0.03, 0.12, n_bumps) * extent * rng.choice([-1.0, 1.0], n_bumps)
+    w = rng.uniform(0.04, 0.15, n_bumps) * extent
+    n_ground = int(n * 0.8)
+    xy = rng.uniform(0, extent, (n_ground, 2))
+    z = (h[None, :] * np.exp(-((xy[:, None, :] - c[None]) ** 2).sum(-1) / (2 * w[None, :] ** 2))).sum(1)
+    ground = np.column_stack([xy, z])
+    n_a = (n - n_ground) // 2
+    u = rng.uniform(0, 1, (n - n_ground, 2))
+    a = u[:n_a]   # tilted plane x = 0.3 extent + 0.4 z, y in [0.1, 0.6] extent
+    pa = np.column_stack([0.3 * extent + 0.12 * extent * a[:, 1], (0.1 + 0.5 * a[:, 0]) * extent, 0.3 * extent * a[:, 1]])
+    b = u[n_a:]   # tilted plane y = 0.75 extent - 0.32 z, x in [0.45, 0.95] extent
+    pb = np.column_stack([(0.45 + 0.5 * b[:, 0]) * extent, 0.75 * extent - 0.08 * extent * b[:, 1], 0.25 * extent * b[:, 1]])
+    return np.concatenate([ground, pa, pb]).astype(np.float32)

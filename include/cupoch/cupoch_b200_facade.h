@@ -901,5 +901,70 @@ inline std::shared_ptr<Feature<33>> ComputeFPFHFeature(const geometry::PointClou
                                                  max_nn, feature->data_.data(), nullptr));
     return feature;
 }
+
+/// registration::FastGlobalRegistrationOption (fast_global_registration.h:43-104)
+class FastGlobalRegistrationOption {
+public:
+    FastGlobalRegistrationOption(float division_factor = 1.4, bool use_absolute_scale = false, bool decrease_mu = true,
+                                 float maximum_correspondence_distance = 0.025, int iteration_number = 64,
+                                 float tuple_scale = 0.95, int maximum_tuple_count = 1000)
+        : division_factor_(division_factor), use_absolute_scale_(use_absolute_scale), decrease_mu_(decrease_mu),
+          maximum_correspondence_distance_(maximum_correspondence_distance), iteration_number_(iteration_number),
+          tuple_scale_(tuple_scale), maximum_tuple_count_(maximum_tuple_count) {}
+    float division_factor_;
+    bool use_absolute_scale_;
+    bool decrease_mu_;
+    float maximum_correspondence_distance_;
+    int iteration_number_;
+    float tuple_scale_;
+    int maximum_tuple_count_;
+    cphb_fgr_option to_c() const {
+        cphb_fgr_option o;
+        o.division_factor = division_factor_;
+        o.use_absolute_scale = use_absolute_scale_ ? 1 : 0;
+        o.decrease_mu = decrease_mu_ ? 1 : 0;
+        o.maximum_correspondence_distance = maximum_correspondence_distance_;
+        o.iteration_number = iteration_number_;
+        o.tuple_scale = tuple_scale_;
+        o.maximum_tuple_count = maximum_tuple_count_;
+        return o;
+    }
+};
+
+/// registration::FastGlobalRegistration<Dim> (fast_global_registration.cu:391-431), Dim = 33 (FPFH) or 352 (SHOT)
+template <int Dim>
+inline RegistrationResult FastGlobalRegistration(const geometry::PointCloud &source, const geometry::PointCloud &target,
+                                                 const Feature<Dim> &source_feature, const Feature<Dim> &target_feature,
+                                                 const FastGlobalRegistrationOption &option = FastGlobalRegistrationOption()) {
+    static_assert(Dim == 33 || Dim == 352, "FastGlobalRegistration supports Feature<33> and Feature<352>");
+    if (source.points_.empty() || target.points_.empty() || source_feature.Num() == 0 || target_feature.Num() == 0) {
+        utility::LogError("Invalid source or target pointcloud.");  // :400-404
+        return RegistrationResult();
+    }
+    cphb_cloud sc = source.view(), tc = target.view();
+    const cphb_fgr_option o = option.to_c();
+    cphb_icp_result r;
+    CorrespondenceSet corr(source.points_.size());
+    utility::check(cphb_fast_global_registration(&sc, &tc, source_feature.data_.data(), source_feature.Num(),
+                                                 target_feature.data_.data(), target_feature.Num(), Dim, &o, &r,
+                                                 reinterpret_cast<int32_t *>(corr.data()), nullptr, nullptr));
+    return to_result(r, std::move(corr));
+}
 }  // namespace registration
+
+namespace knn {
+/// knn::BruteForceNN<Dim>(ref, query, indices, distances) (bruteforce_nn.inl:101-135).  ref / query hold one row of
+/// Dim floats per point (the layout of registration::Feature<Dim>::data_); exact, without a distance matrix.
+template <int Dim>
+inline void BruteForceNN(const utility::device_vector<float> &ref, const utility::device_vector<float> &query,
+                         utility::device_vector<int> &indices, utility::device_vector<float> &distances) {
+    static_assert(Dim == 33 || Dim == 352, "BruteForceNN supports Dim 33 and 352");
+    const size_t nq = query.size() / Dim;
+    indices.resize(nq);
+    distances.resize(nq);
+    if (nq == 0) return;
+    utility::check(cphb_feature_nn(ref.data(), ref.size() / Dim, query.data(), nq, Dim, reinterpret_cast<int32_t *>(indices.data()),
+                                   distances.data(), nullptr, nullptr, nullptr));
+}
+}  // namespace knn
 }  // namespace cupoch

@@ -362,6 +362,52 @@ int cphb_evaluate_registration(const cphb_cloud *source, const cphb_cloud *targe
                                cphb_icp_result *h_result, int32_t *corr_out, void *stream);
 
 /* ------------------------------------------------------------------------ *
+ * Global registration: registration::FastGlobalRegistration
+ * (fast_global_registration.h:43-104, fast_global_registration.cu) and
+ * knn::BruteForceNN (bruteforce_nn.h).  Features are device [n][dim] float32
+ * rows, dim 33 (FPFH) or 352 (SHOT, supplied by the caller).
+ * ------------------------------------------------------------------------ */
+typedef struct cphb_fgr_option { /* FastGlobalRegistrationOption, fast_global_registration.h:55-68 */
+    float division_factor;                 /* 1.4 */
+    int use_absolute_scale;                /* 0 */
+    int decrease_mu;                       /* 1 */
+    float maximum_correspondence_distance; /* 0.025 */
+    int iteration_number;                  /* 64 */
+    float tuple_scale;                     /* 0.95 */
+    int maximum_tuple_count;               /* 1000 (pairs, not triplets) */
+} cphb_fgr_option;
+void cphb_fgr_default_option(cphb_fgr_option *option);
+
+/* knn::BruteForceNN<dim>(ref, query, indices, distances) (bruteforce_nn.inl:101-135): for every query row the
+ * nearest ref row (smallest index among equal distances) and its squared distance, exact, without the reference's
+ * n_ref x n_query distance matrix.  ref_idx_out / ref_d2_out (optional, device, n_ref): also the nearest query row of
+ * every ref row -- the reverse direction, taken from the same distance evaluations (the matcher FastGlobalRegistration
+ * runs).  CPHB_ERR_INVALID for dim other than 33 / 352, an empty set on one side of a requested direction, or a
+ * non-finite feature (found by the kernel; the outputs are then undefined).  Synchronises. */
+int cphb_feature_nn(const float *ref, size_t n_ref, const float *query, size_t n_query, int dim, int32_t *idx_out,
+                    float *d2_out, int32_t *ref_idx_out, float *ref_d2_out, void *stream);
+
+/* Test hook: NormalizePointCloud + AdvancedMatching (fast_global_registration.cu:103-265) on raw clouds and features.
+ * pairs_out (device, 2 * maximum_tuple_count int32) receives the final (source, target) pair list; h_counts =
+ * {pairs written, mutual matches, tuple trials, pairs of passing trials before truncation}.  Synchronises. */
+int cphb_fgr_advanced_matching(const float *source_points, size_t n_source, const float *target_points, size_t n_target,
+                               const float *source_features, size_t n_source_features, const float *target_features,
+                               size_t n_target_features, int dim, const cphb_fgr_option *option, int32_t *pairs_out,
+                               int64_t h_counts[4], void *stream);
+
+/* registration::FastGlobalRegistration<dim> (fast_global_registration.cu:391-431): matching, the graduated
+ * non-convexity pose loop in one device block, then EvaluateRegistration on the original clouds.  corr_out as in
+ * cphb_evaluate_registration; trace_T (device, optional, iteration_number * 16 floats): the normalised pose after
+ * every iteration; h_result->loop_ms is the device time of the pose loop (CUDA events), iterations the updates
+ * applied (0 with fewer than 10 pairs).  A feature count other than the point count, dim other than 33 / 352 (both before any launch)
+ * and non-finite features are CPHB_ERR_INVALID; empty clouds or features give the default result (identity,
+ * fitness 0) and CPHB_OK, as the reference's LogError + RegistrationResult().  Synchronises. */
+int cphb_fast_global_registration(const cphb_cloud *source, const cphb_cloud *target, const float *source_features,
+                                  size_t n_source_features, const float *target_features, size_t n_target_features,
+                                  int dim, const cphb_fgr_option *option, cphb_icp_result *h_result, int32_t *corr_out,
+                                  float *trace_T, void *stream);
+
+/* ------------------------------------------------------------------------ *
  * Host-buffer convenience used by bench.py's e2e leg and the Python mirror:
  * thin wrappers that cudaMalloc/cudaMemcpyAsync around the calls above.
  * ------------------------------------------------------------------------ */
